@@ -1,5 +1,7 @@
+import os
 import sys
-sys.path[:0]=['/root/repo','/root/repo/lfd-a-light-and-fast-detector_b200','/root/repo/tests']
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path[:0] = [os.path.dirname(HERE), os.path.join(os.path.dirname(HERE), 'lfd-a-light-and-fast-detector_b200'), HERE]
 import torch
 from helpers import synth_model
 import synth

@@ -162,6 +162,19 @@ def forward_case(R, name, n, h, w, cls_bias, out_dir):
     print('forward %s: P=%d cls %s loss %s' % (name, cls.shape[1], tuple(cls.shape), ld['loss_values']))
 
 
+def reference_nms_case(nms_ext, out_dir):
+    """The reference's compiled CPU NMS (nms_cpu.cpp) on seeded random boxes, kept indices per (box set, IoU threshold)."""
+    rng = np.random.RandomState(3)
+    cases = []
+    for n in (1, 7, 300):
+        d = np.concatenate([rng.uniform(0, 100, (n, 2)), rng.uniform(1, 40, (n, 2)), rng.uniform(0, 1, (n, 1))], 1).astype(np.float32)
+        d[:, 2:4] += d[:, 0:2]
+        for thr in (0.3, 0.6):
+            cases.append(dict(dets=d, thr=thr, keep=nms_ext.nms(torch.from_numpy(d), thr).numpy()))
+    torch.save(cases, os.path.join(out_dir, 'reference_nms.pt'))
+    print('reference nms: kept %s' % [len(c['keep']) for c in cases])
+
+
 def main():
     R = import_reference()
     out_dir = os.path.join(HERE, 'golden')
@@ -184,6 +197,7 @@ def main():
     torch.save(dict(nms_doc_dets=dets, nms_doc_keep=keep, nms_rand_dets=rnd, nms_rand_keep=keep_rnd, nms_rand_thr=0.3,
                     overlaps_b1=b1, overlaps_b2=b2, overlaps=bbox_overlaps(b1, b2)), os.path.join(out_dir, 'known_answers.pt'))
     print('known answers: doc keep', keep.tolist(), 'random keep', len(keep_rnd))
+    reference_nms_case(R['nms_ext'], out_dir)
 
     for name, (n, h, w, cls_bias) in FORWARD_CASES.items():
         forward_case(R, name, n, h, w, cls_bias, out_dir)
